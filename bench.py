@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- pod x throttle admission checks/sec of the batched throttle-admission pass.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2] [--l2 rotate|flush]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config C2] [--l2 rotate|flush] [--dump-outputs DIR]
   (N>1: python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...)
 
 A "step" is ONE pass of the hot path over one synthetic snapshot: reconcile every throttle against the
@@ -55,7 +55,43 @@ def parse_args():
                     help="how every timed pass gets cold inputs: rotate through enough snapshot copies to exceed L2 twice over (back-to-back "
                          "launches, one event pair) or flush L2 between steps (512 MiB write + 512 MiB read, per-step event pairs)")
     ap.add_argument("--no-extras", action="store_true", help="headline workload only: skip the `configs` array")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed (the pass result a caller receives) to DIR/<name>.npy "
+                         "as float64, under 64 MB in all; rank 0 only")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
+
+
+DUMP_LIMIT = 60_000_000  # bytes of array data per dump: with the .npy headers, under 64 MB
+THROTTLE_FIELDS = ("used", "used_present", "used_cnt", "throttled", "calc_thr", "calc_present", "calc_cnt", "override_active")
+POD_FIELDS = {"running": ("run_bitmap",), "pending": ("pend_bitmap", "codes", "admit")}
+
+
+def dump_outputs(out_dir, res):
+    """Write a PassResult as float64 .npy files, one per field.  The per-throttle columns are written whole.  The per-pod arrays
+    are written whole when everything fits in DUMP_LIMIT bytes; otherwise every array of one pod kind keeps the same seeded
+    sample of rows, and the row numbers go to running_rows.npy / pending_rows.npy.  Bitmap and code words are 32-bit, so
+    float64 holds them exactly; so does it hold the int64 sums below 2^53."""
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {f: getattr(res, f) for f in THROTTLE_FIELDS}
+    fixed = 8 * sum(a.size for a in arrays.values())
+    rows = {kind: getattr(res, fields[0]).shape[0] for kind, fields in POD_FIELDS.items()}
+    row_bytes = {kind: 8 * sum(getattr(res, f)[:1].size for f in fields) for kind, fields in POD_FIELDS.items()}
+    whole = sum(rows[k] * row_bytes[k] for k in POD_FIELDS)
+    if fixed + whole <= DUMP_LIMIT:
+        for fields in POD_FIELDS.values():
+            arrays.update({f: getattr(res, f) for f in fields})
+    else:
+        frac = (DUMP_LIMIT - fixed) / sum(rows[k] * (row_bytes[k] + 8) for k in POD_FIELDS)  # + 8: the row number itself
+        rng = np.random.default_rng(0)
+        for kind, fields in POD_FIELDS.items():
+            pick = np.sort(rng.choice(rows[kind], int(rows[kind] * frac), replace=False))
+            arrays[kind + "_rows"] = pick
+            arrays.update({f: getattr(res, f)[pick] for f in fields})
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, dtype=np.float64))
 
 
 def measured_peaks():
@@ -197,9 +233,11 @@ def run_reference(args, rank, world):
     steps, warm = max(1, args.steps), max(0, args.warmup)
     times = []
     for i in range(warm + steps):
-        _, tm = ko.object_evaluate(snap, threads=threads)
+        res, tm = ko.object_evaluate(snap, threads=threads)
         if i >= warm:
             times.append(tm["total_s"])
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, res)
     med = statistics.median(times)
     checks = snap.pending.n * snap.m
     value = checks / med
@@ -677,6 +715,8 @@ def main():
     t_wall = time.perf_counter() - t_wall0
     clocks = sampler.stop() if rank == 0 else None
     bench.restore_stdout()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, engines[(args.steps - 1) % len(engines)].download())  # the context of the last timed pass
     eng = engines[0]
     Wp = eng.words_per_row
     launches_per_step = head["launches_per_step"]
